@@ -25,6 +25,14 @@ One "step" = one pass of the hot path over the whole per-GPU batch.
            compared with the device's record (bit-exact); a mismatch fails the run.
   cpu_baseline : the reference's own compiled hot path (oracle/_ref) on the host cores, bounded sample, rank 0 at
            N=1 only.
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0's shard), as float64 .npy files:
+  matches[2]   : the match records (adapter, astart, astop, rstart, rstop, score, errors, info per slot) of a fixed,
+                 seeded sample of DUMP_SAMPLE reads, shape [sample, slots, 8]; "2" = the second mate (config 4)
+  qtrim[2]     : the quality-trimming interval of the same reads (config 4)
+  statistics[2]: the whole statistics vector of the step (after the all-reduce)
+  read_index   : which reads the sample holds
+The inputs depend on the arguments only, so two builds can be compared file by file.
 """
 import argparse
 import json
@@ -53,6 +61,8 @@ CONFIG_TEXT = {
     5: "demultiplexing, 96 anchored 5' barcodes with indels (device index), e=0.1",
 }
 HOST_WINDOW_READS = 20_000_000           # pinned host window streamed repeatedly in the e2e leg
+DUMP_SAMPLE = 1 << 18                    # reads in --dump-outputs: at most 44 MB of float64 for any configuration
+DUMP_SEED = 20240923
 
 
 # ------------------------------------------------------------------------------------------------
@@ -384,6 +394,29 @@ def parity_check(config, mates, results, stride=1000):
     return checked, mismatches
 
 
+def dump_outputs(out_dir, mates, results, all_stats):
+    """--dump-outputs: the step's results as float64 .npy files (see the module docstring)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = results[0].n_reads
+    index = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_SAMPLE, replace=False))
+    idx = torch.from_numpy(index).to(results[0].matches.device)
+    arrays = {"read_index": index}
+    pos = 0
+    for k, (m, res) in enumerate(zip(mates, results)):
+        suffix = "2" if k else ""
+        arrays["matches" + suffix] = res.matches.view(n, -1, 8)[idx].cpu().numpy()
+        if res.qtrim is not None:
+            arrays["qtrim" + suffix] = res.qtrim[idx].cpu().numpy()
+        arrays["statistics" + suffix] = all_stats[pos:pos + m["stats"].numel()].cpu().numpy()
+        pos += m["stats"].numel()
+    assert sum(a.size for a in arrays.values()) * 8 <= 64 << 20
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -398,7 +431,11 @@ def main():
                     help="weak: --reads per GPU (default); strong: --reads in total, split evenly over the GPUs")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, a fixed sample of reads)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     cfg = args.config
     if not args.reads:
         args.reads = DEFAULT_READS[cfg]
@@ -539,6 +576,8 @@ def main():
     reads_per_step = n * reads_per_unit
     value = reads_per_step * world * args.steps / (elapsed_ms / 1000.0)
     jit = [m["batch"].adapter_set.jit_status() for m in mates]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, mates, results, all_stats)
 
     # ---- parity of the timed batch: a fixed 1-in-1000 sample against the oracle (outside the timed region) -----
     checked, mismatches = parity_check(cfg, mates, results)
@@ -615,9 +654,7 @@ def main():
         host_ctx.host_profile(reset=True)
         l0 = host_ctx.launch_count()
         t0 = time.perf_counter()
-        # all --steps, and at least 3e8 reads in the timed region: a step of a small configuration (25 M reads) lasts
-        # 50 ms, which one scheduling hiccup of a host thread would double
-        e2e_steps = max(1, args.steps, -(-300_000_000 // max(1, reads_per_step)))
+        e2e_steps = args.steps
         for _ in range(e2e_steps):
             e2e_step()
         barrier()

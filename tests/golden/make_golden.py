@@ -2,14 +2,14 @@
 """
 Generate the golden fixtures under tests/golden/ from the REFERENCE ITSELF.
 
-Run in the build container only (needs /root/reference, builds oracle/_ref on the fly):
+Needs the reference checkout (builds oracle/_ref on the fly):
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [fixture function ...]      (default: all of them)
 
 Everything written here is input/output pairs of the reference's own compiled code
 (cutadapt._align, _kmer_finder, qualtrim, kmer_heuristic, adapters) plus the per-read
 coordinates of the reference's golden files tests/cut/illumina.info.txt and
-illumina5.info.txt.  The fixtures travel to the GPU box, where /root/reference does not exist.
+illumina5.info.txt, so that the tests need neither the reference nor oracle/_ref.
 Seeds are fixed; re-running reproduces the files byte for byte.
 """
 import gzip
@@ -20,8 +20,9 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, ROOT)
+sys.path[:0] = [ROOT, os.path.dirname(HERE)]
 from oracle import build_ref  # noqa: E402
+from util import batch_digest, canon, digest, random_locate_cases  # noqa: E402
 
 build_ref.import_ref()
 from cutadapt._align import Aligner, PrefixComparer, SuffixComparer, edit_environment  # noqa: E402
@@ -466,15 +467,178 @@ def tables():
     dump("tables.json.gz", out)
 
 
+# ---- the reference's answers for the tests that compared with the reference itself ----------------------------------
+
+GATE_READS = 100_000      # reads compared with the reference per configuration in tests/test_gpu_gate.py
+GATE_SAMPLE = 10_000      # of which the answers are stored; the rest are pinned by a digest
+
+
+def reference_suite_kat():
+    """Every call the reference's own tests/test_kmer_heuristic.py makes into cutadapt.kmer_heuristic, with the
+    reference's result, per test (replayed against this package by tests/test_reference_suite.py)."""
+    import pytest
+    from cutadapt import kmer_heuristic as KH
+
+    tests, current, depth = [], [None], [0]
+
+    def recorded(name, fn):
+        def call(*args, **kwargs):
+            depth[0] += 1
+            try:
+                result = fn(*args, **kwargs)
+            finally:
+                depth[0] -= 1
+            if depth[0] == 0 and current[0] is not None:
+                current[0]["calls"].append([name, list(args), kwargs, canon(result)])
+            return result
+        return call
+
+    for name in ("kmer_chunks", "minimize_kmer_search_list", "create_back_overlap_searchsets", "create_positions_and_kmers"):
+        setattr(KH, name, recorded(name, getattr(KH, name)))
+
+    class Recorder:
+        @pytest.hookimpl(hookwrapper=True)
+        def pytest_runtest_call(self, item):
+            mark = item.get_closest_marker("timeout")
+            current[0] = {"test": item.name, "timeout": mark.args[0] if mark else None, "calls": []}
+            yield
+            tests.append(current[0])
+            current[0] = None
+
+    path = os.path.join(REF_TESTS, "test_kmer_heuristic.py")
+    assert pytest.main([path, "-q", "--noconftest", "-p", "no:cacheprovider"], plugins=[Recorder()]) == 0
+    assert all(t["calls"] for t in tests)
+    dump("reference_suite_kat.json.gz", {"test_kmer_heuristic.py": tests})
+
+
+def reference_random_kat():
+    """Aligner.locate and quality_trim_index of the reference on tests/util.py's random_locate_cases()."""
+    answers = []
+    cases = list(random_locate_cases())
+    for ref, rate, flags, wr, wq, ic, mo, queries, qs in cases:
+        al = Aligner(ref, rate, flags, wr, wq, ic, mo)
+        locs = [al.locate(q) for q in queries]
+        answers.append([[list(r) if r else None for r in locs], list(quality_trim_index(qs, 5, 20))])
+    dump("reference_random_kat.json.gz", {"cases_digest": digest(cases), "answers": answers})
+
+
+def _index_rows(idx, reads):
+    rows = []
+    for r in reads:
+        m = idx.match_to(r)
+        rows.append(None if m is None else [int(m.adapter.name[2:]), m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors])
+    return rows
+
+
+def index_reference_kat():
+    """IndexedPrefixAdapters of the 96 barcodes of configuration 5, with and without indels: the keys of its index and
+    its matches on 3000 reads of the configuration (every 50th with an N in the barcode)."""
+    from cutadapt_b200.configs import config5_barcodes, make_config_batch, to_strings
+
+    bcs = config5_barcodes()
+    b = make_config_batch(5, 3000, seed=77)
+    b["seq"][::50, 3] = ord("N")
+    out = {"reads_digest": batch_digest(b)}
+    for key, indels in (("indels", True), ("hamming", False)):
+        idx = RA.IndexedPrefixAdapters([RA.PrefixAdapter(s, max_errors=0.1, indels=indels, name=f"bc{i}")
+                                        for i, s in enumerate(bcs)])
+        out[key] = {"keys": sorted(idx._index._index), "lengths": list(idx._index._lengths),
+                    "rows": _index_rows(idx, to_strings(b["seq"]))}
+    dump("index_reference_kat.json.gz", out)
+
+
+def gate_reference_kat():
+    """The reference's matches on the first GATE_READS reads (configuration 4: GATE_READS / 2 pairs) of each benchmark
+    configuration, drawn on the CPU: the first GATE_SAMPLE answers and the digest of all of them."""
+    from cutadapt.qualtrim import quality_trim_index as qtrim
+    from cutadapt_b200 import configs as CF
+
+    def coords(m):
+        return None if m is None else [m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors]
+
+    def entry(rows):
+        return {"digest": digest(rows), "sample": rows[:GATE_SAMPLE]}
+
+    out = {}
+    for cfg in (2, 3, 4, 5):
+        e = CF.CONFIG_ERROR_RATE[cfg]
+        b = CF.make_config_batch(cfg, GATE_READS // 2 if cfg == 4 else GATE_READS, device="cpu")
+        reads = CF.to_strings(b["seq"])
+        res = {"n": len(reads), "reads_digest": batch_digest(b)}
+        if cfg == 2:
+            ra = RA.BackAdapter(CF.CONFIG2_ADAPTER, max_errors=e, min_overlap=3, name="adapter")
+            res["seq"] = entry([coords(ra.match_to(r)) for r in reads])
+        elif cfg == 3:
+            objs = [RA.BackAdapter(s, max_errors=e, min_overlap=3, name=f"a{i}") for i, s in enumerate(CF.CONFIG3_BACK)]
+            objs.append(RA.LinkedAdapter(RA.PrefixAdapter(CF.CONFIG3_LINKED[0], max_errors=e, min_overlap=3, name="lf"),
+                                         RA.BackAdapter(CF.CONFIG3_LINKED[1], max_errors=e, min_overlap=3, name="lb"),
+                                         True, False, "linked"))
+            rmulti = RA.MultipleAdapters(objs)
+            res["seq"] = entry([match_desc(rmulti.match_to(r)) for r in reads])
+        elif cfg == 4:
+            for skey, qkey, adapter in (("seq", "qual", CF.CONFIG4_R1), ("seq2", "qual2", CF.CONFIG4_R2)):
+                ra = RA.BackAdapter(adapter, max_errors=e, min_overlap=3, name="x")
+                rows = []
+                for r, q in zip(CF.to_strings(b[skey]), CF.to_strings(b[qkey])):
+                    s, t = qtrim(q, 0, 20, 33)
+                    rows.append([s, t, coords(ra.match_to(r[s:t]))])
+                res[skey] = entry(rows)
+        else:
+            idx = RA.IndexedPrefixAdapters([RA.PrefixAdapter(s, max_errors=e, min_overlap=3, indels=True, name=f"bc{i}")
+                                            for i, s in enumerate(CF.config5_barcodes())])
+            res["seq"] = entry(_index_rows(idx, reads))
+        out[str(cfg)] = res
+    dump("gate_reference_kat.json.gz", out)
+
+
+def parity_reference_kat():
+    """BackAdapter AGATCGGAAGAGC (e = 0.1) of the reference on the first 3000 reads of make_reads(10000, config=1)
+    (tests/test_gpu_parity.py)."""
+    from cutadapt_b200.synth import make_reads
+
+    reads = make_reads(10000, config=1)[0][:3000]
+    ra = RA.BackAdapter("AGATCGGAAGAGC", max_errors=0.1, name="a")
+    rows = []
+    for read in reads:
+        m = ra.match_to(read)
+        rows.append(None if m is None else [m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors])
+    dump("parity_reference_kat.json.gz", {"reads_digest": digest(reads), "rows": rows})
+
+
+def statistics_reference_kat():
+    """The reference's AdapterStatistics fed with its own matches on the reads of tests/_dist_worker.workload()
+    (the four adapters built there): per adapter and end, errors as [length, errors, count] and adjacent_bases."""
+    from _dist_worker import workload
+
+    reads, _ = workload()
+    robjs = [RA.BackAdapter("AGATCGGAAGAGC", max_errors=0.1, name="a"), RA.FrontAdapter("ACGTTGCATTGAC", max_errors=0.1, name="f"),
+             RA.AnywhereAdapter("CTGTCTCTTATACACATCT", max_errors=0.1, name="w"),
+             RA.LinkedAdapter(RA.PrefixAdapter("GTTCAGAGTTCTACAGTCCGACGATC", max_errors=0.1, name="lf"),
+                              RA.BackAdapter("TGGAATTCTCGGGTGCCAAGG", max_errors=0.1, name="lb"), False, False, "linked")]
+    rmulti = RA.MultipleAdapters(robjs)
+    rstats = {id(a): a.create_statistics() for a in robjs}
+    for read in reads:
+        m = rmulti.match_to(read)
+        if m is not None:
+            rstats[id(m.adapter)].add_match(m)
+    adapters = []
+    for a in robjs:
+        ends = []
+        for end in rstats[id(a)].end_statistics():
+            ends.append(None if end is None else {
+                "errors": sorted([length, e, n] for length, d in end.errors.items() for e, n in d.items()),
+                "adjacent_bases": sorted([base, n] for base, n in end.adjacent_bases.items())})
+        adapters.append(ends)
+    dump("statistics_reference_kat.json.gz", {"reads_digest": digest(reads), "adapters": adapters})
+
+
+FIXTURES = [locate_kat, comparer_kat, kmer_kat, qualtrim_kat, trim_scans_kat, adapters_kat, index_kat, info_file_kat,
+            env_kat, dp_debug_kat, tables, reference_suite_kat, reference_random_kat, index_reference_kat,
+            gate_reference_kat, parity_reference_kat, statistics_reference_kat]
+
+
 if __name__ == "__main__":
-    locate_kat()
-    comparer_kat()
-    kmer_kat()
-    qualtrim_kat()
-    trim_scans_kat()
-    adapters_kat()
-    index_kat()
-    info_file_kat()
-    env_kat()
-    dp_debug_kat()
-    tables()
+    wanted = sys.argv[1:]
+    for fn in FIXTURES:
+        if not wanted or fn.__name__ in wanted:
+            fn()

@@ -68,27 +68,19 @@ def test_two_rank_statistics_allreduce(tmp_path):
                 assert ea.errors == eb.errors and ea.adjacent_bases == eb.adjacent_bases, a.name
     lay = stats_layout(len(spec.adapters), 200, 3)
     assert (r0[lay["lengths"]:lay["lengths"] + 201] == lengths).all()
-    # against the reference itself, where it travelled along: its AdapterStatistics fed with its own matches
-    from util import reference_or_none
+    # against the reference itself: its AdapterStatistics fed with its own matches (statistics_reference_kat)
+    from util import digest, golden
 
-    if reference_or_none() is not None:
-        import cutadapt.adapters as RA
-
-        robjs = [RA.BackAdapter("AGATCGGAAGAGC", max_errors=0.1, name="a"), RA.FrontAdapter("ACGTTGCATTGAC", max_errors=0.1, name="f"),
-                 RA.AnywhereAdapter("CTGTCTCTTATACACATCT", max_errors=0.1, name="w"),
-                 RA.LinkedAdapter(RA.PrefixAdapter("GTTCAGAGTTCTACAGTCCGACGATC", max_errors=0.1, name="lf"),
-                                  RA.BackAdapter("TGGAATTCTCGGGTGCCAAGG", max_errors=0.1, name="lb"), False, False, "linked")]
-        rmulti = RA.MultipleAdapters(robjs)
-        rstats = {id(a): a.create_statistics() for a in robjs}
-        for read in reads:
-            m = rmulti.match_to(read)
-            if m is not None:
-                rstats[id(m.adapter)].add_match(m)
-        for mine, robj in zip(rebuilt, robjs):
-            for ea, eb in zip(mine.end_statistics(), rstats[id(robj)].end_statistics()):
-                assert (ea is None) == (eb is None)
-                if ea is not None:
-                    assert ea.errors == {k: dict(v) for k, v in eb.errors.items() if v} and ea.adjacent_bases == eb.adjacent_bases
+    g = golden("statistics_reference_kat.json.gz")
+    assert digest(reads) == g["reads_digest"] and len(g["adapters"]) == len(rebuilt)
+    for mine, ends in zip(rebuilt, g["adapters"]):
+        for ea, eb in zip(mine.end_statistics(), ends):
+            assert (ea is None) == (eb is None)
+            if ea is not None:
+                errors = {}
+                for length, e, count in eb["errors"]:
+                    errors.setdefault(length, {})[e] = count
+                assert ea.errors == errors and ea.adjacent_bases == dict(eb["adjacent_bases"]), mine.name
     # the FASTQ counters of both ranks add up to the single-process totals
     import json
     from oracle import oracle

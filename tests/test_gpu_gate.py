@@ -1,15 +1,16 @@
 """
 Parity at the gate BASELINE.md states: >= 10^6 synthetic reads per benchmark configuration against the C oracle
 (oracle_process_packed: the oracle's per-read pass as one C loop, run from all host threads) and >= 10^5 against
-the reference itself (oracle/_ref, the reference compiled in the build container, when it travelled along).
-The reads are the generators of cutadapt_b200.configs (SURVEY.md section 8(d)).
+the reference itself.  The reads are the generators of cutadapt_b200.configs (SURVEY.md section 8(d)).  The
+reference's answers are stored (tests/golden/gate_reference_kat.json.gz, made by make_golden.py): they belong to the
+first 10^5 reads each generator draws on the CPU, so that part of each test trims reads drawn on the CPU.
 """
 import numpy as np
 import pytest
 
 from cutadapt_b200 import _lib as L
 from oracle import oracle
-from util import reference_or_none, build_adapters, match_desc
+from util import batch_digest, digest, golden, match_desc
 
 pytestmark = pytest.mark.gpu
 
@@ -29,22 +30,31 @@ def _packed(t):
     return host, np.arange(n + 1, dtype=np.int64) * L_
 
 
-def _reference_records(ref_multi, reads, quals=None, cutoff=None):
-    """(astart, astop, rstart, rstop, score, errors) or None per read from the compiled reference."""
-    from cutadapt.qualtrim import quality_trim_index
+def _coords(rec):
+    return None if rec["adapter"] < 0 else [int(rec[f]) for f in ("astart", "astop", "rstart", "rstop", "score", "errors")]
 
-    out = []
-    for i, r in enumerate(reads):
-        if cutoff is not None:
-            s, e = quality_trim_index(quals[i], 0, cutoff, 33)
-            r = r[s:e]
-        m = ref_multi.match_to(r)
-        out.append(match_desc(m))
-    return out
+
+def _reference_batch(config):
+    """The reads the stored reference answers of `config` belong to."""
+    from cutadapt_b200.configs import make_config_batch
+
+    ref = golden("gate_reference_kat.json.gz")[str(config)]
+    assert ref["n"] == (N_REF // 2 if config == 4 else N_REF)
+    b = make_config_batch(config, ref["n"], device="cpu")
+    assert batch_digest(b) == ref["reads_digest"], "the generator no longer draws the reads the answers belong to"
+    return b
+
+
+def _assert_reference_rows(config, key, rows):
+    """One row per read against the reference's: row by row over the stored sample, all rows through the digest."""
+    ref = golden("gate_reference_kat.json.gz")[str(config)][key]
+    for i, (have, want) in enumerate(zip(rows, ref["sample"])):
+        assert have == want, (config, key, i)
+    assert digest(rows) == ref["digest"], (config, key, "differs from the reference after the stored sample")
 
 
 def test_gate_config2_one_adapter():
-    from cutadapt_b200.configs import config_adapters, make_config_batch, to_strings
+    from cutadapt_b200.configs import config_adapters, make_config_batch
 
     multi, _ = config_adapters(2)
     descs, groups = _flat(multi)
@@ -55,21 +65,12 @@ def test_gate_config2_one_adapter():
     exp, _ = oracle.oracle_process_packed(descs, groups, data, offsets)
     assert (got == exp).all()
     assert 0.45 < (got["adapter"][:, 0, 0] >= 0).mean() < 0.56
-    ref = reference_or_none()
-    if ref is not None:
-        import cutadapt.adapters as RA
-
-        ra = RA.BackAdapter("AGATCGGAAGAGC", max_errors=0.1, min_overlap=3, name="adapter")
-        reads = to_strings(seq[:N_REF])
-        for read, rec in zip(reads, got[:N_REF, 0, 0]):
-            m = ra.match_to(read)
-            want = None if m is None else (m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors)
-            have = None if rec["adapter"] < 0 else tuple(int(rec[f]) for f in ("astart", "astop", "rstart", "rstop", "score", "errors"))
-            assert want == have, read
+    got, _ = aset.process(*_packed(_reference_batch(2)["seq"]))
+    _assert_reference_rows(2, "seq", [_coords(rec) for rec in got[:, 0, 0]])
 
 
 def test_gate_config3_five_adapters():
-    from cutadapt_b200.configs import config_adapters, make_config_batch, to_strings, CONFIG3_BACK, CONFIG3_LINKED
+    from cutadapt_b200.configs import config_adapters, make_config_batch, to_strings
 
     multi, _ = config_adapters(3)
     descs, groups = _flat(multi)
@@ -85,28 +86,20 @@ def test_gate_config3_five_adapters():
     grp = got["info"][:, 0, :].max(axis=1) & 255
     for g in range(5):
         assert (hit & (grp == g)).mean() > 0.03, g
-    ref = reference_or_none()
-    if ref is not None:
-        import cutadapt.adapters as RA
-
-        objs = [RA.BackAdapter(s, max_errors=0.15, min_overlap=3, name=f"a{i}") for i, s in enumerate(CONFIG3_BACK)]
-        objs.append(RA.LinkedAdapter(RA.PrefixAdapter(CONFIG3_LINKED[0], max_errors=0.15, min_overlap=3, name="lf"),
-                                     RA.BackAdapter(CONFIG3_LINKED[1], max_errors=0.15, min_overlap=3, name="lb"),
-                                     True, False, "linked"))
-        rmulti = RA.MultipleAdapters(objs)
-        reads = to_strings(seq[:N_REF])
-        for i, read in enumerate(reads):
-            assert match_desc(multi.matches_from_records(got[i, 0], read)) == match_desc(rmulti.match_to(read)), read
+    seq = _reference_batch(3)["seq"]
+    got, _ = aset.process(*_packed(seq))
+    _assert_reference_rows(3, "seq", [match_desc(multi.matches_from_records(got[i, 0], read))
+                                      for i, read in enumerate(to_strings(seq))])
 
 
 def test_gate_config4_pairs_with_quality_trimming():
-    from cutadapt_b200.configs import config_adapters, make_config_batch, to_strings, CONFIG4_R1, CONFIG4_R2
+    from cutadapt_b200.configs import config_adapters, make_config_batch
 
     m1, m2 = config_adapters(4)
     n_pairs = N_GATE // 2
     b = make_config_batch(4, n_pairs, device="cuda")
-    ref = reference_or_none()
-    for multi, skey, qkey, adapter in ((m1, "seq", "qual", CONFIG4_R1), (m2, "seq2", "qual2", CONFIG4_R2)):
+    rb = _reference_batch(4)
+    for multi, skey, qkey in ((m1, "seq", "qual"), (m2, "seq2", "qual2")):
         descs, groups = _flat(multi)
         data, offsets = _packed(b[skey])
         qdata, _ = _packed(b[qkey])
@@ -116,26 +109,15 @@ def test_gate_config4_pairs_with_quality_trimming():
         exp, eqt = oracle.oracle_process_packed(descs, groups, data, offsets, qdata, True, 0, 20)
         assert (gqt == eqt).all() and (got == exp).all(), skey
         assert 0.4 < (got["adapter"][:, 0, 0] >= 0).mean() < 0.6
-        if ref is not None:
-            import cutadapt.adapters as RA
-            from cutadapt.qualtrim import quality_trim_index
-
-            ra = RA.BackAdapter(adapter, max_errors=0.1, min_overlap=3, name="x")
-            reads, quals = to_strings(b[skey][:N_REF // 2]), to_strings(b[qkey][:N_REF // 2])
-            for i, (read, q) in enumerate(zip(reads, quals)):
-                s, e = quality_trim_index(q, 0, 20, 33)
-                assert (s, e) == tuple(gqt[i])
-                m = ra.match_to(read[s:e])
-                want = None if m is None else (m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors)
-                rec = got[i, 0, 0]
-                have = None if rec["adapter"] < 0 else tuple(int(rec[f]) for f in ("astart", "astop", "rstart", "rstop", "score", "errors"))
-                assert want == have, (skey, read)
+        data, offsets = _packed(rb[skey])
+        got, gqt = aset.process(data, offsets, _packed(rb[qkey])[0], params)
+        _assert_reference_rows(4, skey, [[int(s), int(e), _coords(rec)] for (s, e), rec in zip(gqt, got[:, 0, 0])])
 
 
 def test_gate_config5_barcode_index_with_indels():
     """96 anchored 5' barcodes, e = 0.1 with indels: the device index against the oracle's own index (built from the
     oracle's edit environment) on 10^6 reads, and against the reference's IndexedPrefixAdapters."""
-    from cutadapt_b200.configs import config_adapters, config5_barcodes, make_config_batch, to_strings
+    from cutadapt_b200.configs import config_adapters, config5_barcodes, make_config_batch
 
     multi, _ = config_adapters(5)
     seq = make_config_batch(5, N_GATE, device="cuda")["seq"]
@@ -150,19 +132,6 @@ def test_gate_config5_barcode_index_with_indels():
     for f in ("astart", "astop", "rstart", "rstop", "score", "errors"):
         assert (got[f][:, 0, 0] == exp[f]).all(), f
     assert 0.95 < (got["adapter"][:, 0, 0] >= 0).mean() < 0.995
-    ref = reference_or_none()
-    if ref is not None:
-        import cutadapt.adapters as RA
-
-        idx = RA.IndexedPrefixAdapters([RA.PrefixAdapter(b, max_errors=0.1, min_overlap=3, indels=True, name=f"bc{i}")
-                                        for i, b in enumerate(barcodes)])
-        names = {f"bc{i}": i for i in range(len(barcodes))}
-        reads = to_strings(seq[:N_REF])
-        for i, read in enumerate(reads):
-            m = idx.match_to(read)
-            rec = got[i, 0, 0]
-            if m is None:
-                assert rec["adapter"] < 0, read
-            else:
-                assert (names[m.adapter.name], m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors) == \
-                    tuple(int(rec[f]) for f in ("adapter", "astart", "astop", "rstart", "rstop", "score", "errors")), read
+    got, _ = aset.process(*_packed(_reference_batch(5)["seq"]))
+    _assert_reference_rows(5, "seq", [None if rec["adapter"] < 0 else [int(rec["adapter"])] + _coords(rec)
+                                      for rec in got[:, 0, 0]])

@@ -1,14 +1,13 @@
 """
 The oracle against the reference: every function of oracle/cutadapt_oracle.c is pinned to the
-golden vectors generated from the reference's own compiled code (tests/golden/make_golden.py)
-and, where oracle/_ref travels along, to the reference itself on fresh random inputs.
+golden vectors generated from the reference's own compiled code (tests/golden/make_golden.py).
 """
 import random
 
 import pytest
 
 from oracle import oracle
-from util import golden, reference_or_none, match_desc, build_adapters
+from util import batch_digest, digest, golden, match_desc, build_adapters, random_locate_cases
 
 
 def test_locate_golden():
@@ -72,30 +71,16 @@ def test_info_file_coordinates():
     assert n_hits > 30
 
 
-@pytest.mark.skipif(reference_or_none() is None, reason="oracle/_ref not built (needs /root/reference)")
 def test_against_reference_random():
-    import cutadapt._align as ra
-    from cutadapt.qualtrim import quality_trim_index
-
-    rng = random.Random(77)
-    for _ in range(3000):
-        alpha = rng.choice(["ACGT", "AC", "ACGTN", "ACGTacgtNn", "ACGTRYKMN"])
-        m = rng.randint(1, 20)
-        ref = "".join(rng.choice(alpha) for _ in range(m))
-        wr, wq = rng.random() < 0.3, rng.random() < 0.2
-        if wr and set(ref.upper()) <= {"N"}:
-            continue
-        rate = rng.choice([0, 0.1, 0.2, 0.34, 0.5])
-        flags, ic, mo = rng.randint(0, 15), rng.choice([1, 1, 100000, 3]), rng.randint(1, 4)
-        al = ra.Aligner(ref, rate, flags, wr, wq, ic, mo)
-        for _ in range(4):
-            q = "".join(rng.choice(alpha) for _ in range(rng.randint(0, 40)))
-            if rng.random() < 0.5:
-                pos = rng.randint(0, len(q))
-                q = q[:pos] + ref[rng.randint(0, m // 2):] + q[pos:]
-            assert al.locate(q) == oracle.locate(ref, q, rate, flags, wr, wq, ic, mo), (ref, q, rate, flags)
-        qs = "".join(chr(33 + rng.choice([0, 2, 10, 20, 30, 40])) for _ in range(rng.randint(0, 50)))
-        assert quality_trim_index(qs, 5, 20) == oracle.quality_trim_index(qs, 5, 20)
+    """Aligner.locate / quality_trim_index of the reference on 3000 random cases (answers: reference_random_kat)."""
+    g = golden("reference_random_kat.json.gz")
+    cases = list(random_locate_cases())
+    assert digest(cases) == g["cases_digest"] and len(cases) == len(g["answers"])
+    for (ref, rate, flags, wr, wq, ic, mo, queries, qs), (locs, qt) in zip(cases, g["answers"]):
+        for q, expected in zip(queries, locs):
+            got = oracle.locate(ref, q, rate, flags, wr, wq, ic, mo)
+            assert (list(got) if got is not None else None) == expected, (ref, q, rate, flags)
+        assert list(oracle.quality_trim_index(qs, 5, 20)) == qt, qs
 
 
 def test_oracle_composition_matches_golden_adapters():
@@ -231,35 +216,29 @@ def test_packed_batch_loop_equals_the_per_read_composition():
 
 
 def test_neighbourhoods_and_index_golden():
-    """edit_environment / hamming_sphere / AdapterIndex of the oracle against the reference's own (goldens + _ref)."""
+    """edit_environment / hamming_sphere / AdapterIndex of the oracle against the reference's own (goldens)."""
     for t, k, ee, he in golden("environment_kat.json.gz"):
         assert sorted(map(list, oracle.edit_environment(t, k))) == sorted(ee), (t, k)
         ham = [[s, e, len(t) - e] for e in range(k + 1) for s in oracle.hamming_sphere(t, e)]
         assert sorted(ham) == sorted(he), (t, k)
-    ref = reference_or_none()
-    if ref is None:
-        return
     import numpy as np
-    import cutadapt.adapters as RA
     import cutadapt_b200.adapters as PA
     from cutadapt_b200.configs import config5_barcodes, make_config_batch, to_strings
 
+    # the reference's IndexedPrefixAdapters of the 96 barcodes: index keys and matches (index_reference_kat)
+    g = golden("index_reference_kat.json.gz")
     bcs = config5_barcodes()
-    for indels in (True, False):
+    b = make_config_batch(5, 3000, seed=77)
+    b["seq"][::50, 3] = ord("N")
+    assert batch_digest(b) == g["reads_digest"]
+    for key, indels in (("indels", True), ("hamming", False)):
         lengths, index = oracle.index_build(bcs, 0.1, indels)
-        idx = RA.IndexedPrefixAdapters([RA.PrefixAdapter(b, max_errors=0.1, indels=indels, name=f"bc{i}") for i, b in enumerate(bcs)])
-        assert set(idx._index._index) == set(index) and list(idx._index._lengths) == lengths
-        seq = make_config_batch(5, 3000, seed=77)["seq"]
-        seq[::50, 3] = ord("N")
-        host = seq.numpy().reshape(-1)
+        assert sorted(index) == g[key]["keys"] and lengths == g[key]["lengths"]
+        host = b["seq"].numpy().reshape(-1)
         offs = np.arange(3001, dtype=np.int64) * 150
-        descs = [PA.PrefixAdapter(b, max_errors=0.1, indels=indels, name=f"bc{i}").descriptor() for i, b in enumerate(bcs)]
+        descs = [PA.PrefixAdapter(s, max_errors=0.1, indels=indels, name=f"bc{i}").descriptor() for i, s in enumerate(bcs)]
         out = oracle.oracle_index_process(bcs, 0.1, indels, True, host, offs, descs)
-        for i, r in enumerate(to_strings(seq)):
-            m = idx.match_to(r)
-            rec = out[i]
-            if m is None:
-                assert rec["adapter"] < 0
-            else:
-                assert (int(m.adapter.name[2:]), m.astart, m.astop, m.rstart, m.rstop, m.score, m.errors) == tuple(
-                    int(rec[f]) for f in ("adapter", "astart", "astop", "rstart", "rstop", "score", "errors")), r
+        for r, rec, expected in zip(to_strings(b["seq"]), out, g[key]["rows"]):
+            have = None if rec["adapter"] < 0 else [
+                int(rec[f]) for f in ("adapter", "astart", "astop", "rstart", "rstop", "score", "errors")]
+            assert have == expected, (key, r)

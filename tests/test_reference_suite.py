@@ -1,39 +1,30 @@
 """
-The reference's OWN test files run against this package (where the reference checkout is mounted: the build
-container; skipped on the GPU box, which has no /root/reference).  A shim maps the module names the tests import
-(``cutadapt.kmer_heuristic``, ``cutadapt._match_tables`` ...) onto cutadapt_b200's modules; nothing of the
-reference is copied or imported.  Only the host-side modules can be exercised here -- the tests of the aligner,
-the k-mer finder and the adapter classes call into the GPU library and the GPU box has no reference checkout;
-their known answers are part of tests/golden/ (make_golden.py) and run there through the library.
+The reference's OWN test files replayed against this package.  tests/golden/make_golden.py ran each file against the
+reference and recorded, per test, every call it made into the module under test with the reference's result (and
+the test's time limit, if it has one); here the same calls go to cutadapt_b200's module and must give the same
+results.  Results are compared as the reference's tests compare them: lists and sets without regard to order
+(util.canon).  Only host-side modules are covered here -- the aligner, the k-mer finder and the adapter classes run
+on the GPU library; their known answers are the other fixtures of tests/golden/.
 """
-import os
-import subprocess
-import sys
+import importlib
+import time
 
 import pytest
 
-REF_TESTS = "/root/reference/tests"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from util import canon, golden
 
-SHIM = r'''
-import sys, types
-sys.path.insert(0, {root!r})
-import cutadapt_b200.kmer_heuristic as kh
-import cutadapt_b200._match_tables as mt
-pkg = types.ModuleType("cutadapt")
-pkg.__path__ = []
-sys.modules["cutadapt"] = pkg
-sys.modules["cutadapt.kmer_heuristic"] = kh
-sys.modules["cutadapt._match_tables"] = mt
-import pytest
-sys.exit(pytest.main([{path!r}, "-q", "--noconftest", "-p", "no:cacheprovider"] + {extra!r}))
-'''
+KAT = golden("reference_suite_kat.json.gz")
+MODULES = {"test_kmer_heuristic.py": "cutadapt_b200.kmer_heuristic"}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="reference checkout not mounted")
-@pytest.mark.parametrize("name,extra", [("test_kmer_heuristic.py", [])])
-def test_reference_test_file_passes_against_this_package(name, extra):
-    code = SHIM.format(root=ROOT, path=os.path.join(REF_TESTS, name), extra=extra)
-    proc = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert proc.returncode == 0, proc.stdout[-3000:] + proc.stderr[-2000:]
-    assert " passed" in proc.stdout
+@pytest.mark.parametrize("name", sorted(KAT))
+def test_reference_test_file_passes_against_this_package(name):
+    module = importlib.import_module(MODULES[name])
+    tests = KAT[name]
+    assert len(tests) >= 15
+    for test in tests:
+        t0 = time.perf_counter()
+        for fn, args, kwargs, expected in test["calls"]:
+            assert canon(getattr(module, fn)(*args, **kwargs)) == expected, (test["test"], fn, args, kwargs)
+        if test["timeout"] is not None:
+            assert time.perf_counter() - t0 < test["timeout"], test["test"]

@@ -1,6 +1,7 @@
 """Shared helpers of the test-suite (test infrastructure only)."""
 import ctypes as C
 import gzip
+import hashlib
 import json
 import os
 import random
@@ -16,22 +17,53 @@ def golden(name):
         return json.load(f)
 
 
-def reference_or_none():
-    """The reference's compiled hot path (oracle/_ref), if it has been built and travels along."""
-    import sys
+def digest(obj):
+    """sha256 of the compact JSON form of `obj` (numpy integers count as ints): lets a fixture pin a list of answers
+    too long to store."""
+    return hashlib.sha256(json.dumps(obj, separators=(",", ":"), default=int).encode()).hexdigest()
 
-    ref_root = os.path.join(ROOT, "oracle", "_ref")
-    if not os.path.isdir(os.path.join(ref_root, "cutadapt")):
-        return None
-    if ref_root not in sys.path:
-        sys.path.insert(0, ref_root)
-    try:
-        import cutadapt.adapters  # noqa: F401
-        import cutadapt
 
-        return cutadapt
-    except Exception:
-        return None
+def batch_digest(batch):
+    """sha256 of the reads (and qualities) of a make_config_batch() result: pins the generator a fixture was made with."""
+    h = hashlib.sha256()
+    for key in ("seq", "qual", "seq2", "qual2"):
+        if batch.get(key) is not None:
+            h.update(np.ascontiguousarray(batch[key].cpu().numpy()).tobytes())
+    return h.hexdigest()
+
+
+def canon(x):
+    """A result in a form that ignores the order of lists and sets but keeps the order inside tuples."""
+    if isinstance(x, tuple):
+        return [canon(v) for v in x]
+    if isinstance(x, (list, set, frozenset)):
+        return sorted((canon(v) for v in x), key=json.dumps)
+    return x
+
+
+def random_locate_cases():
+    """(reference, max_error_rate, flags, wildcard_ref, wildcard_query, indel_cost, min_overlap, [4 queries],
+    qualities) of the random oracle-against-reference test; tests/golden/reference_random_kat.json.gz holds the
+    reference's answers."""
+    rng = random.Random(77)
+    for _ in range(3000):
+        alpha = rng.choice(["ACGT", "AC", "ACGTN", "ACGTacgtNn", "ACGTRYKMN"])
+        m = rng.randint(1, 20)
+        ref = "".join(rng.choice(alpha) for _ in range(m))
+        wr, wq = rng.random() < 0.3, rng.random() < 0.2
+        if wr and set(ref.upper()) <= {"N"}:
+            continue
+        rate = rng.choice([0, 0.1, 0.2, 0.34, 0.5])
+        flags, ic, mo = rng.randint(0, 15), rng.choice([1, 1, 100000, 3]), rng.randint(1, 4)
+        queries = []
+        for _ in range(4):
+            q = "".join(rng.choice(alpha) for _ in range(rng.randint(0, 40)))
+            if rng.random() < 0.5:
+                pos = rng.randint(0, len(q))
+                q = q[:pos] + ref[rng.randint(0, m // 2):] + q[pos:]
+            queries.append(q)
+        qs = "".join(chr(33 + rng.choice([0, 2, 10, 20, 30, 40])) for _ in range(rng.randint(0, 50)))
+        yield ref, rate, flags, wr, wq, ic, mo, queries, qs
 
 
 # ---- hostsim: the device functions compiled for the host (tests only) ------------------------
